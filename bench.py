@@ -3,6 +3,7 @@
   python bench.py [--gpus N] [--steps K] [--warmup W] [--precision P] [--workload W]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...      # the reference's CPU path (oracle port)
+  python bench.py --dump-outputs DIR ...    # also write the last timed step's outputs as .npy
 
 Metric (BASELINE.json): ray-samples/sec, coarse+fine, device-timed; PSNR vs ref.
 One ray-sample = one (warp MLP + NeRF MLP) point evaluation; a ray costs
@@ -108,7 +109,56 @@ def parse_args():
   ap.add_argument('--no-cpu-baseline', action='store_true')
   ap.add_argument('--no-parity', action='store_true')
   ap.add_argument('--cpu-seconds', type=float, default=15.0)
-  return ap.parse_args()
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                  help='after the timed steps, write what the last timed step returned (rank 0) '
+                       'as DIR/<name>.npy')
+  args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl != 'b200':
+    ap.error('--dump-outputs writes the outputs of the b200 arm')
+  return args
+
+
+DUMP_MAX_BYTES = 60 * 2**20      # the .npy files of one dump stay under 64 MB together
+
+
+def dump_outputs(out_dir, arrays):
+  """Writes {name: tensor} as out_dir/<name>.npy (float32, or float64 where the tensor is).
+  Inputs are seeded, so two builds' dumps of the same command compare element for element.
+  Above DUMP_MAX_BYTES in all, every array keeps the same fixed, seeded sample of its
+  leading dimension (arrays with the same leading size keep the same rows)."""
+  import numpy as np
+  import torch
+  arrays = {k: v.detach().cpu().to(torch.float64 if v.dtype == torch.float64 else torch.float32)
+            for k, v in arrays.items()}
+  total = sum(v.numel() * v.element_size() for v in arrays.values())
+  if total > DUMP_MAX_BYTES:
+    keep = DUMP_MAX_BYTES / total
+    for k, v in arrays.items():
+      if v.dim() == 0:
+        continue
+      n = v.shape[0]
+      idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:max(1, int(n * keep))]
+      arrays[k] = v[idx.sort().values]
+  os.makedirs(out_dir, exist_ok=True)
+  for k, v in arrays.items():
+    np.save(os.path.join(out_dir, k + '.npy'), v.numpy())
+
+
+def flat_outputs(tree, prefix=''):
+  """{'coarse': {'rgb': t, ...}, ...} -> {'coarse_rgb': t, ...} (tensor and number leaves; '/' -> '_')."""
+  import torch
+  flat = {}
+  for k, v in tree.items():
+    name = prefix + k.replace('/', '_')
+    if isinstance(v, dict):
+      flat.update(flat_outputs(v, name + '_'))
+    elif torch.is_tensor(v):
+      flat[name] = v
+    elif isinstance(v, (int, float)):
+      flat[name] = torch.tensor(float(v), dtype=torch.float64)
+  return flat
 
 
 def oracle_spec(wl):
@@ -604,6 +654,7 @@ def measure(precision, wl, B, args, ctx, want_parity):
       'value': world * B * evals / (ms_per_step * 1e-3),
       'launches': int(launches), 'clocks': clocks, 'wall': wall,
       'field_ms': (statistics.mean(m[0] for m in field_ms), statistics.mean(m[1] for m in field_ms)),
+      'out': out,
   }
   if want_parity and rank == 0:
     res['parity'] = parity_check(model, variables, params_cpu, rays_host, out, wl, precision)
@@ -656,11 +707,11 @@ def roofline(res, wl, B, peaks, precision):
   return r
 
 
-def measure_eval_frame(args, wl, precision, ctx, steps):
+def measure_eval_frame(args, wl, precision, ctx, steps, dump_dir=None):
   """BASELINE.json's fifth config (eval.py:330-353): a full frame, rays split
   1 -> N GPUs, forward only.  A step = one frame through
   nerfies_b200.evaluation.render_frame; the collective's time is reported.
-  Returns the JSON line (rank 0) or None."""
+  Returns the JSON line (rank 0) or None; dump_dir receives the last frame."""
   import numpy as np
   import torch
   import torch.distributed as dist
@@ -709,6 +760,8 @@ def measure_eval_frame(args, wl, precision, ctx, steps):
   gather_ms = float(tot[1]) / steps
   if rank != 0:
     return None
+  if dump_dir:
+    dump_outputs(dump_dir, flat_outputs(frame))
   value = w * h * evals / (ms * 1e-3)
   line = {
       'metric': 'ray-samples/sec (coarse+fine, device-timed)', 'value': value,
@@ -807,6 +860,10 @@ def measure_train_step(args, wl, ctx):
     dist.all_reduce(tot, op=dist.ReduceOp.MAX)
   if rank != 0:
     return None
+  if args.dump_outputs:
+    opt = state.optimizer
+    dump_outputs(args.dump_outputs, {'params': opt.flat, 'adam_m': opt.m, 'adam_v': opt.v,
+                                     **flat_outputs(stats)})
   ms = float(tot[0]) / args.steps
   n_params = state.optimizer.flat.numel()
   return {
@@ -862,13 +919,15 @@ def run_b200(args):
       dist.destroy_process_group()
     return
   if 'frame' in wl:
-    line = measure_eval_frame(args, wl, precision, ctx, args.steps)
+    line = measure_eval_frame(args, wl, precision, ctx, args.steps, dump_dir=args.dump_outputs)
     if rank == 0:
       emit(line)
     if world > 1:
       dist.destroy_process_group()
     return
   main = measure(precision, wl, B, args, ctx, want_parity=not args.no_parity)
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, flat_outputs(main['out']))
 
   # End to end through the C ABI's host entry point: host buffers in, host
   # buffers out, H2D + D2H inside the timed region.

@@ -187,11 +187,21 @@ def test_cta_pair_variant_is_bit_identical(monkeypatch):
   weight unit, one issuer feeds both SMs) computes the same per-row arithmetic, so
   its outputs equal the default tcgen05 kernel's bit for bit - including ragged
   sizes where the follower CTA's tile lies beyond the end.  The release library reads
-  no environment variables: this runs only against a developer build
-  (`python tools/build_variant.py dev -DNFB_DEV_KNOBS`, loaded through NFB_LIB_PATH)."""
+  no environment variables: against it, this test reruns itself in a subprocess that
+  loads the -DNFB_DEV_KNOBS developer build which build() makes (through NFB_LIB_PATH)."""
+  import os, subprocess, sys
   from nerfies_b200 import _lib
   if 'libnfb_dev' not in _lib.LIB_PATH:
-    pytest.skip('needs the -DNFB_DEV_KNOBS developer build (NFB_LIB_PATH=nerfies_b200/_variants/libnfb_dev.so)')
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dev_lib = os.path.join(root, 'nerfies_b200', '_variants', 'libnfb_dev.so')
+    assert os.path.exists(dev_lib), f'{dev_lib} is missing: run __graft_entry__.build()'
+    out = subprocess.run(
+        [sys.executable, '-m', 'pytest', '-q', '-p', 'no:cacheprovider',
+         os.path.abspath(__file__) + '::test_cta_pair_variant_is_bit_identical'],
+        cwd=root, env=dict(os.environ, NFB_LIB_PATH=dev_lib), capture_output=True, text=True,
+        timeout=600)
+    assert out.returncode == 0 and '1 passed' in out.stdout, (out.stdout[-3000:], out.stderr[-2000:])
+    return
   spec = O.OracleSpec(num_coarse_samples=128, num_fine_samples=128, near=0.02, far=0.83,
                       num_nerf_point_freqs=8, sigma_activation='softplus', use_warp=True,
                       use_appearance_metadata=True, num_warp_embeddings=9,

@@ -3,13 +3,11 @@
   python tools/build_variant.py epidbg -DNFB_EPI_DEBUG
   NFB_LIB_PATH=nerfies_b200/_variants/libnfb_epidbg.so python bench.py ...
 """
-import os, subprocess, sys
+import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import __graft_entry__ as g
 
 name, defs = sys.argv[1], sys.argv[2:]
-out_dir = os.path.join(g.REPO, 'nerfies_b200', '_variants')
-os.makedirs(out_dir, exist_ok=True)
-out = os.path.join(out_dir, 'libnfb_%s.so' % name)
-subprocess.run(['nvcc'] + g.NVCC_FLAGS + ['-DNFB_WITH_TC'] + defs + ['-o', out, os.path.join(g.CSRC, 'nfb_api.cu')], check=True, cwd=g.REPO)
+out = os.path.join(g.REPO, 'nerfies_b200', '_variants', 'libnfb_%s.so' % name)
+g._compile(out, ['-DNFB_WITH_TC'] + defs, force=True)
 print(out)
