@@ -197,7 +197,13 @@ int nfb_warp_forward(nfb_handle* h, int num_points, const float* points,
  *   grads[i]: device tensor of the i-th parameter of nfb_param_info, rows*cols floats,
  *             ACCUMULATED into (+=): zero them first for a plain gradient;
  *   loss_out (device, 2 floats): the coarse and the fine loss.
- * The 'glo' warp metadata encoder only; NFB_FLAG_METADATA_ENCODED is not supported. */
+ * Every warp metadata encoder trains; NFB_FLAG_METADATA_ENCODED is not supported.  `warp_id`:
+ *   'glo'   (B) uint32 GLO ids;
+ *   'time'  (B) float32 metadata['time'], as for nfb_render_forward (reinterpreted pointer);
+ *   'blend' (B) uint32 GLO ids; the TimeEncoder sees float(id).
+ * The 'time' / 'blend' encoders read warp_extra['time_alpha'] from nfb_set_time_alpha: the
+ * TimeEncoder's window is cosine_easing_window(F, time_alpha) for 'time' and fully open for
+ * 'blend', whose embedding is (1 - time_alpha) glo + time_alpha time (warping.py:128-133). */
 int nfb_train_value_and_grad(nfb_handle* h, int num_rays, const float* origins,
                              const float* directions, const float* viewdirs,
                              const unsigned* warp_id, const unsigned* appearance_id,
@@ -219,7 +225,9 @@ typedef struct nfb_train_reg {
   int use_background_loss;         /* training.py:146 */
   int num_background_points;
   const float* background_points;        /* device (P,3): batch['background_points'] */
-  const unsigned* background_warp_ids;   /* device (P): the reference draws random.choice(key, model.warp_ids) */
+  const unsigned* background_warp_ids;   /* device (P) uint32 ids for EVERY encoder: the reference draws
+                                            random.choice(key, model.warp_ids) and the 'time' encoder sees
+                                            float(id) with alpha = time_alpha (training.py:121-131) */
   const float* background_noise;         /* device (P,3) or NULL: noise_std * random.normal(key, points.shape) */
   float background_loss_weight;          /* ScalarParams.background_loss_weight */
 } nfb_train_reg;
@@ -242,7 +250,9 @@ int nfb_train_value_and_grad_reg(nfb_handle* h, int B, const float* origins, con
 
 /* Jacobian of the warp field at free points: jacobian_out (P,3,3), J[i][j] = d warped_i / d point_j
  * (jax.jacfwd(self.warp, argnums=0), warping.py:196-198, 385-387); warped_out (P,3) nullable.
- * warp_id (P) GLO ids.  fp32, any precision mode of the handle (layer-wise tape kernels). */
+ * warp_id (P) as for nfb_warp_forward: GLO ids, float32 timestamps for the 'time' encoder; the metadata
+ * embedding is a constant of the Jacobian.  The warp MLP must use relu.  fp32, any precision mode of the
+ * handle (layer-wise tape kernels). */
 int nfb_warp_jacobian(nfb_handle* h, int P, const float* points, const unsigned* warp_id, float warp_alpha,
                       float* warped_out, float* jacobian_out, void* stream);
 

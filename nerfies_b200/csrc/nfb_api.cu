@@ -308,8 +308,27 @@ int launch_check(nfb_handle* h, const char* what) {
   return 0;
 }
 
+// The TimeEncoder's window: cosine_easing_window(F, alpha) (modules.py:274-294) with alpha =
+// time_alpha for 'time' and F for 'blend' (alpha = None, modules.py:318-319, warping.py:131).
+void time_window(const nfb_handle* h, float* w) {
+  const int F = h->cfg.time_encoder_num_freqs;
+  const float alpha = h->cfg.warp_metadata_encoder == NFB_WARP_ENC_TIME ? h->time_alpha : (float)F;
+  const float pi = 3.14159274101257324f;
+  for (int k = 0; k < F; ++k) {
+    float x = alpha - (float)k;
+    x = fminf(fmaxf(x, 0.f), 1.f);
+    volatile float arg = pi * x;
+    arg = arg + pi;
+    volatile float cv = cosf(arg);
+    w[k] = 0.5f * (1.f + cv);
+  }
+}
+
+// time_from_ids: `warp_id` holds uint32 ids even for the 'time' encoder, whose TimeEncoder then sees
+// float(id) - the background points of the training loss (training.py:121-131).
 int run_cond(nfb_handle* h, int B, const float* viewdirs, const unsigned* warp_id,
-             const unsigned* app_id, const unsigned* cam_id, cudaStream_t s, bool encoded = false) {
+             const unsigned* app_id, const unsigned* cam_id, cudaStream_t s, bool encoded = false,
+             bool time_from_ids = false) {
   const nfb_config& c = h->cfg;
   nfb::CondArgs a{};
   a.viewdirs = viewdirs; a.warp_id = warp_id; a.app_id = app_id; a.cam_id = cam_id;
@@ -324,26 +343,17 @@ int run_cond(nfb_handle* h, int B, const float* viewdirs, const unsigned* warp_i
   if (h->prog[0].G + h->prog[0].tc + h->prog[0].ac + h->prog[0].rc == 0) return 0;
   const long long total = (long long)B * a.stride;
   const int enc = c.warp_field_type != NFB_WARP_NONE ? c.warp_metadata_encoder : NFB_WARP_ENC_GLO;
-  if (enc == NFB_WARP_ENC_TIME && !encoded) a.warp_id = nullptr;   // `warp_id` carries float timestamps
+  if (enc == NFB_WARP_ENC_TIME && !encoded) a.warp_id = nullptr;   // no GLO table; `warp_id` may carry timestamps
   nfb::ray_cond_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(a);
   if (launch_check(h, "ray_cond_kernel")) return -1;
   if (enc != NFB_WARP_ENC_GLO && !encoded && warp_id) {
-    // TimeEncoder on metadata['time'] ('time') or on float(id) ('blend', alpha = None)
+    // TimeEncoder on metadata['time'] ('time') or on float(id) ('blend'; 'time' with time_from_ids)
     nfb::TimeArgs t{};
     t.params = h->d_packed; t.net = h->time_net;
     t.F = c.time_encoder_num_freqs;
-    if (enc == NFB_WARP_ENC_TIME) t.time_f = reinterpret_cast<const float*>(warp_id);
+    if (enc == NFB_WARP_ENC_TIME && !time_from_ids) t.time_f = reinterpret_cast<const float*>(warp_id);
     else t.time_id = warp_id;
-    const float alpha = enc == NFB_WARP_ENC_TIME ? h->time_alpha : (float)t.F;   // modules.py:318-319
-    const float pi = 3.14159274101257324f;
-    for (int k = 0; k < t.F; ++k) {                     // cosine_easing_window (modules.py:274-294)
-      float x = alpha - (float)k;
-      x = fminf(fmaxf(x, 0.f), 1.f);
-      volatile float arg = pi * x;
-      arg = arg + pi;
-      volatile float cv = cosf(arg);
-      t.window[k] = 0.5f * (1.f + cv);
-    }
+    time_window(h, t.window);
     t.blend = enc == NFB_WARP_ENC_BLEND; t.time_alpha = h->time_alpha;
     t.cond = h->d_cond; t.stride = h->cond_stride; t.G = h->prog[0].G; t.num_rays = B;
     nfb::time_embed_kernel<<<(B + nfb::kTimeRays - 1) / nfb::kTimeRays, nfb::kTimeThreads, 0, s>>>(t);
@@ -772,7 +782,7 @@ void nfb_destroy(nfb_handle* h) {
                    h->d_wc, h->d_samples, h->d_out_c, h->d_out_f, h->d_in};
   for (float* p : bufs) if (p) cudaFree(p);
   float* tbufs[] = {h->d_tape, h->d_gpacked, h->d_gwarp, h->d_gapp, h->d_gcam, h->d_dcond, h->d_tr_out, h->d_tr_w, h->d_loss,
-                    h->d_ttape, reinterpret_cast<float*>(h->d_sel)};
+                    h->d_ttape, reinterpret_cast<float*>(h->d_sel), h->d_time_tape};
   for (float* p : tbufs) if (p) cudaFree(p);
   if (h->d_ids) cudaFree(h->d_ids);
   for (int l = 0; l < 2; ++l)

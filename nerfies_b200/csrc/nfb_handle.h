@@ -97,6 +97,7 @@ struct nfb_handle {
   float *d_dcond = nullptr, *d_tr_out = nullptr, *d_tr_w = nullptr, *d_loss = nullptr;
   float* d_ttape = nullptr; long long ttape_floats = 0;     // tangent tape (train_reg.cuh)
   int* d_sel = nullptr; long long sel_cap = 0;              // selected tape rows (median-depth samples)
+  float* d_time_tape = nullptr; long long time_tape_floats = 0;   // TimeEncoder tape (train_api.cuh)
   int x3_pair_ok = -1;                // fp16x3 CTA-pair launch: -1 unknown, 0 unavailable, n = co-resident clusters
   int debug_bits = 0;                 // FieldArgs::debug bits set through the test hook (abort-path test)
   long long* trace = nullptr;

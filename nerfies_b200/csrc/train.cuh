@@ -586,6 +586,9 @@ struct CondBwdArgs {
   const unsigned* warp_id; const unsigned* app_id; const unsigned* cam_id;
   float* d_warp_table; float* d_app_table; float* d_cam_table;
   int n_warp, n_app, n_cam, G, A, C, Fv, use_viewdirs, use_app, use_cam, use_trunk_c, use_alpha_c;
+  // The warp block [0, G) is a GLO row for 'glo' (scale 1) and 'blend' (scale 1 - time_alpha,
+  // warping.py:132-133).  'time' has no GLO table (warp_glo = 0): its warp_id may hold float timestamps.
+  int warp_glo; float warp_scale;
 };
 __global__ void cond_bwd_kernel(const CondBwdArgs a) {
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -600,9 +603,10 @@ __global__ void cond_bwd_kernel(const CondBwdArgs a) {
     atomicAdd(a.d_app_table + (size_t)id * a.A + j, v);
   };
   if (q < a.G) {
+    if (!a.warp_glo) return;
     unsigned id = a.warp_id ? a.warp_id[ray] : 0u;
     id = min(id, (unsigned)(a.n_warp - 1));
-    atomicAdd(a.d_warp_table + (size_t)id * a.G + q, v);
+    atomicAdd(a.d_warp_table + (size_t)id * a.G + q, a.warp_scale * v);
     return;
   }
   q -= a.G;
@@ -622,6 +626,38 @@ __global__ void cond_bwd_kernel(const CondBwdArgs a) {
     id = min(id, (unsigned)(a.n_cam - 1));
     atomicAdd(a.d_cam_table + (size_t)id * a.C + q, v);
   }
+}
+
+// ---------------------------------------------------------------------------
+// TimeEncoder backward, first stage: per condition vector, the encoder's input row (the input
+// stage of time_embed_kernel, same arithmetic) and the seed dZ of its output layer,
+// seed_scale * dcond[:, 0:G] (1 for 'time', time_alpha for 'blend': warping.py:132-133).  The
+// layers themselves go through the training GEMMs (net_forward / net_backward).
+// ---------------------------------------------------------------------------
+struct TimeTapeArgs {
+  const float* time_f;        // (rows) metadata['time'], or null
+  const unsigned* time_id;    // (rows) ids read as timestamps, float(id), or null
+  int F;                      // metadata_encoder_num_freqs
+  float window[20];           // cosine_easing_window(F, alpha) as run_cond builds it
+  const float* dcond; int cond_stride, G; float seed_scale;
+  float* in; int ld_in;       // (rows, ld_in): [t, w_f sin(2^f t), w_f sin(2^f t + pi/2)]_f
+  float* seed; int ld_seed;   // (rows, ld_seed); the padding columns stay as they are (zero)
+  long long rows;
+};
+__global__ void time_tape_kernel(const __grid_constant__ TimeTapeArgs a) {
+  const long long m = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (m >= a.rows) return;
+  const float t = a.time_f ? a.time_f[m] : (float)a.time_id[m];
+  float* o = a.in + m * a.ld_in;
+  o[0] = t;
+  for (int k = 1; k < 1 + 2 * a.F; ++k) {
+    const int f = (k - 1) >> 1;
+    float ang = t * exp2f((float)f);
+    if ((k - 1) & 1) ang = ang + kHalfPiF;
+    o[k] = a.window[f] * sinf(ang);
+  }
+  const float* g = a.dcond + m * a.cond_stride;
+  for (int q = 0; q < a.G; ++q) a.seed[m * a.ld_seed + q] = a.seed_scale * g[q];
 }
 
 // packed (K x ld, column offset) gradient -> the caller's dense (rows x cols) tensor (+=).

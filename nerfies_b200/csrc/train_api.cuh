@@ -391,11 +391,62 @@ int train_prepare_rows(nfb_handle* h, long long rows) {
   return train_prepare(h, (int)std::max<long long>(1, (rows + smax - 1) / smax));
 }
 
+// The GLO side of the warp block of the condition gradient (CondBwdArgs::warp_glo / warp_scale).
+void set_warp_glo(const nfb_handle* h, nfb::train::CondBwdArgs& a) {
+  const int enc = h->cfg.warp_metadata_encoder;
+  a.warp_glo = enc != NFB_WARP_ENC_TIME;
+  a.warp_scale = enc == NFB_WARP_ENC_BLEND ? 1.f - h->time_alpha : 1.f;
+}
+
+// TimeEncoder backward (modules.py:297-322) for `rows` condition vectors whose warp-block gradient
+// d_dcond[:, 0:G] is complete: the encoder's input rows onto its own tape, its forward recomputed
+// layer-wise, then dW / db accumulated into d_gpacked at the encoder's offsets.  The recomputed
+// activations can differ from time_embed_kernel's in round-off only, so a ReLU mask can differ only
+// on a pre-activation within round-off of zero.  `warp_id` / `time_from_ids` as for run_cond.
+int time_encoder_backward(nfb_handle* h, int rows, const unsigned* warp_id, bool time_from_ids, cudaStream_t s) {
+  using namespace nfb::train;
+  const nfb_config& c = h->cfg;
+  const int enc = c.warp_metadata_encoder;
+  if (c.warp_field_type == NFB_WARP_NONE || enc == NFB_WARP_ENC_GLO || rows == 0) return 0;
+  const Net& net = h->time_net;
+  const int F = c.time_encoder_num_freqs, ld_in = 1 + 2 * F, last = net.n_steps - 1;
+  // input rows, every layer's output, then the gradient region: every layer's dY and the input's
+  // gradient (written by the first layer's dX GEMM, not needed)
+  long long off = 0, out[nfb::kMaxSteps], d_out[nfb::kMaxSteps];
+  auto take = [&](long long n) { long long o = off; off += (n + 63) / 64 * 64; return o; };
+  const long long in = take((long long)rows * ld_in);
+  for (int i = 0; i < net.n_steps; ++i) out[i] = take((long long)rows * net.steps[i].npad);
+  const long long grad_begin = off;
+  for (int i = 0; i < net.n_steps; ++i) d_out[i] = take((long long)rows * net.steps[i].npad);
+  const long long d_in = take((long long)rows * ld_in);
+  if (h->time_tape_floats < off) {
+    if (h->d_time_tape) cudaFree(h->d_time_tape);
+    h->d_time_tape = nullptr; h->time_tape_floats = 0;
+    if (cudaMalloc(&h->d_time_tape, (size_t)off * sizeof(float)) != cudaSuccess)
+      return fail("training: cannot allocate a %.2f GB TimeEncoder tape", off * 4e-9);
+    h->time_tape_floats = off;
+  }
+  float* T = h->d_time_tape;
+  NFB_CUDA(cudaMemsetAsync(T + grad_begin, 0, (size_t)(off - grad_begin) * sizeof(float), s));
+  TimeTapeArgs a{};
+  if (enc == NFB_WARP_ENC_TIME && !time_from_ids) a.time_f = reinterpret_cast<const float*>(warp_id);
+  else a.time_id = warp_id;
+  a.F = F;
+  time_window(h, a.window);
+  a.dcond = h->d_dcond; a.cond_stride = h->cond_stride; a.G = h->prog[0].G;
+  a.seed_scale = enc == NFB_WARP_ENC_BLEND ? h->time_alpha : 1.f;      // warping.py:132-133
+  a.in = T + in; a.ld_in = ld_in; a.seed = T + d_out[last]; a.ld_seed = net.steps[last].npad; a.rows = rows;
+  time_tape_kernel<<<(unsigned)((rows + 127) / 128), 128, 0, s>>>(a);
+  if (launch_check(h, "time_tape_kernel")) return -1;
+  if (net_forward(h, net, T + in, ld_in, out, T, rows, s)) return -1;
+  return net_backward(h, net, T + in, T + d_in, ld_in, out, d_out, T, rows, s);
+}
+
 // warp_field.apply on `n` free points (+ optional noise) on the tape of level 0: condition
 // vectors per point, encoded inputs, warp MLP, tail.  The points land in tape.pts, the warped
-// points in tape.warped.
+// points in tape.warped.  `time_from_ids` as for run_cond.
 int warp_points_forward(nfb_handle* h, int n, const float* points, const float* noise, const unsigned* warp_id,
-                        cudaStream_t s) {
+                        bool time_from_ids, cudaStream_t s) {
   using namespace nfb::train;
   const nfb::FieldProgram& p = h->prog[0];
   const TapeLayout t = tape_layout(p, n);
@@ -403,7 +454,8 @@ int warp_points_forward(nfb_handle* h, int n, const float* points, const float* 
   const unsigned blocks = (unsigned)((n + 127) / 128);
   add_noise_kernel<<<(unsigned)(((long long)n * 3 + 255) / 256), 256, 0, s>>>(points, noise, A + t.warped, (long long)n * 3);
   if (launch_check(h, "add_noise_kernel")) return -1;
-  if (run_cond(h, n, A + t.warped, warp_id, nullptr, nullptr, s)) return -1;      // the "view direction" columns are unused here
+  // the "view direction" columns are unused here
+  if (run_cond(h, n, A + t.warped, warp_id, nullptr, nullptr, s, false, time_from_ids)) return -1;
   EncodeArgs e{};
   e.pts_in = A + t.warped; e.pts_out = A + t.pts; e.cond = h->d_cond; e.window = h->d_window;
   e.in = A + t.in_w; e.F = p.Fw; e.ld = t.ld_w; e.S = 1;
@@ -419,6 +471,8 @@ int warp_points_forward(nfb_handle* h, int n, const float* points, const float* 
 }
 
 // compute_background_loss (training.py:118-135) and its gradient, in chunks of max_rays points.
+// `warp_ids` are uint32 ids for every encoder: the reference draws them from model.warp_ids and
+// hands them to warp_field.apply, so the 'time' encoder sees float(id) (training.py:121-131).
 int train_background(nfb_handle* h, int P, const float* points, const unsigned* warp_ids, const float* noise,
                      float weight, cudaStream_t s) {
   using namespace nfb::train;
@@ -430,7 +484,9 @@ int train_background(nfb_handle* h, int P, const float* points, const unsigned* 
     const int n = std::min(chunk, P - p0);
     const TapeLayout t = tape_layout(p, n);
     float* A = h->d_tape;
-    if (warp_points_forward(h, n, points + (size_t)p0 * 3, noise ? noise + (size_t)p0 * 3 : nullptr, warp_ids + p0, s)) return -1;
+    if (warp_points_forward(h, n, points + (size_t)p0 * 3, noise ? noise + (size_t)p0 * 3 : nullptr, warp_ids + p0,
+                            true, s))
+      return -1;
     NFB_CUDA(cudaMemsetAsync(A + t.grad_begin, 0, (size_t)(t.grad_end - t.grad_begin) * sizeof(float), s));
     NFB_CUDA(cudaMemsetAsync(h->d_dcond, 0, (size_t)n * h->cond_stride * sizeof(float), s));
     // alpha = -2, scale = 0.001: the defaults of compute_background_loss, which train_step does not override
@@ -456,9 +512,11 @@ int train_background(nfb_handle* h, int P, const float* points, const unsigned* 
     a.G = p.G; a.A = c.num_appearance_features; a.C = c.num_camera_features; a.Fv = c.num_nerf_viewdir_freqs;
     a.use_viewdirs = c.use_viewdirs; a.use_app = c.use_appearance_metadata; a.use_cam = c.use_camera_metadata;
     a.use_trunk_c = c.use_trunk_condition; a.use_alpha_c = c.use_alpha_condition;
+    set_warp_glo(h, a);
     const long long total = (long long)n * a.stride;
     cond_bwd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(a);
     if (launch_check(h, "cond_bwd_kernel")) return -1;
+    if (time_encoder_backward(h, n, warp_ids + p0, true, s)) return -1;
   }
   return 0;
 }
@@ -478,8 +536,9 @@ int nfb_train_value_and_grad_reg(nfb_handle* h, int B, const float* origins, con
   if (count != (int)h->specs.size()) return fail("expected %d gradient tensors, got %d", (int)h->specs.size(), count);
   if (flags & NFB_FLAG_METADATA_ENCODED) return fail("training with metadata_encoded=True is not supported");
   const nfb_config& c = h->cfg;
-  if (c.warp_field_type != NFB_WARP_NONE && c.warp_metadata_encoder != NFB_WARP_ENC_GLO)
-    return fail("training supports the 'glo' warp metadata encoder only (no TimeEncoder backward)");
+  const bool time_enc = c.warp_field_type != NFB_WARP_NONE && c.warp_metadata_encoder != NFB_WARP_ENC_GLO;
+  if (time_enc && !(flags & NFB_FLAG_NO_WARP) && !warp_id)
+    return fail("the 'time' / 'blend' warp metadata encoders need warp_id (metadata['time'] / ids)");
   for (int i = 0; i < count; ++i)
     if (numels[i] != h->specs[i].rows * h->specs[i].cols)
       return fail("gradient %d (%s): expected %lld elements", i, h->specs[i].name.c_str(), h->specs[i].rows * h->specs[i].cols);
@@ -552,10 +611,12 @@ int nfb_train_value_and_grad_reg(nfb_handle* h, int B, const float* origins, con
     a.G = h->prog[0].G; a.A = c.num_appearance_features; a.C = c.num_camera_features; a.Fv = c.num_nerf_viewdir_freqs;
     a.use_viewdirs = c.use_viewdirs; a.use_app = c.use_appearance_metadata; a.use_cam = c.use_camera_metadata;
     a.use_trunk_c = c.use_trunk_condition; a.use_alpha_c = c.use_alpha_condition;
+    set_warp_glo(h, a);
     const long long total = (long long)B * a.stride;
     nfb::train::cond_bwd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(a);
     if (launch_check(h, "cond_bwd_kernel")) return -1;
   }
+  if (use_warp && time_encoder_backward(h, B, warp_id, false, s)) return -1;
   // background loss (training.py:118-135, 246-257): warp_field.apply on free points
   const int P = (reg && reg->use_background_loss) ? reg->num_background_points : 0;
   if (P > 0) {
@@ -600,9 +661,7 @@ int nfb_warp_jacobian(nfb_handle* h, int P, const float* points, const unsigned*
   if (!h || !points || !jacobian_out) return fail("null argument");
   if (P < 0) return fail("P must be >= 0");
   if (check_call(h, std::min(P, h->max_rays))) return -1;
-  const nfb_config& c = h->cfg;
   if (h->prog[0].warp_type == 0) return fail("the model has no warp field");
-  if (c.warp_metadata_encoder != NFB_WARP_ENC_GLO) return fail("warp Jacobian: 'glo' warp metadata encoder only");
   cudaStream_t s = (cudaStream_t)stream;
   if (enter_stream(h, s)) return -1;
   if (P == 0) return 0;
@@ -611,7 +670,8 @@ int nfb_warp_jacobian(nfb_handle* h, int P, const float* points, const unsigned*
   if (train_prepare_rows(h, chunk)) return -1;
   for (int p0 = 0; p0 < P; p0 += chunk) {
     const int n = std::min(chunk, P - p0);
-    if (warp_points_forward(h, n, points + (size_t)p0 * 3, nullptr, warp_id ? warp_id + p0 : nullptr, s)) return -1;
+    if (warp_points_forward(h, n, points + (size_t)p0 * 3, nullptr, warp_id ? warp_id + p0 : nullptr, false, s))
+      return -1;
     const nfb::FieldProgram& p = h->prog[0];
     const TapeLayout t = tape_layout(p, n);
     if (warped_out)

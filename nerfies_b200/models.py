@@ -380,8 +380,8 @@ class NerfModel:
         jac_levels.append('coarse')
       if return_warp_jacobian:
         jac_levels.append('fine')
-    if jac_levels and (metadata_encoded or self.warp_metadata_encoder_type != 'glo'):
-      raise NotImplementedError("warp Jacobians: 'glo' warp metadata ids only")
+    if jac_levels and metadata_encoded:
+      raise NotImplementedError('warp Jacobians of metadata_encoded=True calls')
     want_points = return_points
     return_points = return_points or bool(jac_levels)       # the Jacobian is taken at the sample points
     params = variables['params']
@@ -581,8 +581,8 @@ class WarpField:
     non-warp parameters keep their last uploaded values (zeros if none were ever
     uploaded - the warp-only launch does not read them)."""
     m = self.model
-    if return_jacobian and (metadata_encoded or m.warp_metadata_encoder_type != 'glo'):
-      raise NotImplementedError("warp Jacobian: 'glo' warp metadata ids only")
+    if return_jacobian and metadata_encoded:
+      raise NotImplementedError('warp Jacobian of a metadata_encoded=True call')
     dev = m.device
     pts = _prep_f32(points, dev)
     shape = pts.shape

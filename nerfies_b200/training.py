@@ -140,7 +140,15 @@ def value_and_grad(model, params, batch, warp_extra, rngs=None, chunk_rays=256, 
   B = origins.shape[0]
   viewdirs = _prep_f32(batch['viewdirs'], dev) if 'viewdirs' in batch else None
   md = batch.get('metadata', {})
-  warp_id = _prep_ids(md.get('warp'), dev) if model.use_warp else None
+  enc = model.warp_metadata_encoder_type if model.use_warp else None
+  if enc == 'time':
+    # models.py:252-254: the warp field reads metadata['time'] (B,1) float32
+    t = md.get('time')
+    warp_id = None if t is None else _prep_f32(t, dev).reshape(-1)
+  else:
+    warp_id = _prep_ids(md.get('warp'), dev) if model.use_warp else None
+  if enc in ('time', 'blend') and warp_id is None:
+    raise KeyError(f"batch['metadata']['{'time' if enc == 'time' else 'warp'}'] is required")
   app_id = _prep_ids(md.get('appearance'), dev) if model.use_appearance_metadata else None
   cam_id = _prep_ids(md.get('camera'), dev) if model.use_camera_metadata else None
   target = _prep_f32(batch['rgb'], dev)[..., :3].contiguous()
@@ -150,6 +158,7 @@ def value_and_grad(model, params, batch, warp_extra, rngs=None, chunk_rays=256, 
   u_rand = None if u_rand is None else _prep_f32(u_rand, dev)
   hd = model.handle(B)
   hd.set_params(params)
+  model._set_time_alpha(hd, (warp_extra or {}).get('time_alpha'))
   n = len(hd.param_specs)
   numels = [r * c for _, r, c in hd.param_specs]
   if grads is None:
@@ -203,7 +212,8 @@ def train_step(model, rng_key, state, batch, scalar_params, use_elastic_loss=Fal
   if use_elastic_loss or use_warp_reg_loss or use_background_loss:
     bg = {}
     if use_background_loss:
-      # training.py:122-126: ids ~ random.choice(key, model.warp_ids), noise ~ noise_std * N(0, 1)
+      # training.py:122-126: ids ~ random.choice(key, model.warp_ids), noise ~ noise_std * N(0, 1);
+      # integer ids for every encoder ('time' encodes float(id), as the reference does)
       pts = torch.as_tensor(batch['background_points']).reshape(-1, 3)
       gen = torch.Generator().manual_seed(int(rng_key) if not isinstance(rng_key, torch.Generator) else rng_key.seed())
       warp_ids = torch.as_tensor(list(model.warp_ids), dtype=torch.int64)
